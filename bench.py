@@ -67,6 +67,8 @@ def parse_args():
     p.add_argument("--no-verify", action="store_true", help="N > 1: skip the sharded-vs-single-GPU parity check")
     p.add_argument("--large-n", type=int, default=65536, help="env count of roofline_large_n (0 = skip)")
     p.add_argument("--no-neighbours", action="store_true", help="skip the side measurements of the SURVEY 8(f) kernels")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step returned to its caller as DIR/<name>.npy (rank 0)")
     return p.parse_args()
 
 
@@ -345,6 +347,20 @@ def main():
             graph_of(n_)
     run_steps(W)           # warm-up (>= 3 steps)
     stream.synchronize()
+    # the clock-sampler spin-up below runs a time-dependent number of steps: on a state set of its own, so that the timed
+    # steps start from the state the warm-up left and the same arguments give them the same inputs
+    spin = None
+    if use_graph:
+        spare = eng.new_buffers(N)
+        spare.load_logical(make_state(spec, N, seed=1234 + 1000 * S, rank=rank))
+        spare.cmd_uniforms, spare.obs_uniforms = None, [None, None]
+        with torch.cuda.stream(stream):
+            one_step(spare)
+        stream.synchronize()
+        spin = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(spin, stream=stream):
+            for _ in range(G):
+                one_step(spare)
 
     def barrier():
         if world > 1:
@@ -365,7 +381,7 @@ def main():
         if use_graph:
             with torch.cuda.stream(stream):
                 for _ in range(20):
-                    graphs[G].replay()
+                    spin.replay()
             stream.synchronize()
         else:
             time.sleep(0.05)
@@ -378,6 +394,10 @@ def main():
     barrier()
     t_wall = time.perf_counter() - t_wall0
     elapsed_ms = ev0.elapsed_time(ev1)
+    last_outputs = None
+    if args.dump_outputs and rank == 0:   # read now: everything after the timed region steps the same sets again
+        last_set = ((K - 1) % G if use_graph else K - 1) % S
+        last_outputs = step_outputs(spec, sets[last_set])
     if rank == 0 and t_wall < 1.0 and use_graph:
         # nvidia-smi samples every 100 ms: keep the same graphs running (untimed) long enough for the clock record to
         # show the GPU under load
@@ -544,8 +564,42 @@ def main():
             "wall_s_timed_region": t_wall,
         }
         _emit(line)
+    if last_outputs is not None:
+        write_outputs(Path(args.dump_outputs), last_outputs)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6 - 4096   # 64 MB in all, .npy headers included
+
+
+def step_outputs(spec, b) -> tuple[dict, dict]:
+    """What the caller of one env step receives, copied to the host: per-env arrays (observation rows of each group,
+    reward, done masks, the joint targets of the processed action) and the others (reset ids, reset logging means)."""
+    per_env = {f"obs_{grp.name}": b.obs[g] for g, grp in enumerate(spec.obs) if b.obs[g] is not None}
+    per_env.update(reward=b.reward, terminated=b.terminated, truncated=b.truncated, joint_target=b.logical("joint_target"))
+    per_env = {k: v.float().cpu() for k, v in per_env.items()}
+    other = {"reset_ids": b.reset_ids[: int(b.n_reset.item())].double().cpu(), "reset_log": b.log_all.float().cpu()}
+    return per_env, other
+
+
+def write_outputs(out_dir: Path, outputs: tuple[dict, dict]) -> None:
+    """One float32 / float64 .npy file per array. Beyond 64 MB in all, the per-env arrays keep a fixed, seeded sample of
+    env rows, listed in env_ids.npy."""
+    import numpy as np
+
+    per_env, other = outputs
+    n = next(iter(per_env.values())).shape[0]
+    nbytes = sum(v.numel() * v.element_size() for v in per_env.values())
+    budget = DUMP_LIMIT_BYTES - sum(v.numel() * v.element_size() for v in other.values()) - 8 * n
+    if nbytes > budget:
+        keep = n * budget // nbytes
+        ids = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        per_env = {k: v[ids] for k, v in per_env.items()}
+        other = {**other, "env_ids": ids.double()}
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, v in {**per_env, **other}.items():
+        np.save(out_dir / f"{name}.npy", v.contiguous().numpy())
 
 
 def measure_large_n(spec, n_large, dev, rng, roofline_of, stream):

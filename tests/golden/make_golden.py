@@ -121,8 +121,82 @@ def pits():
         print("pit_terrain", key, n, "envs,", int(ref["was_on_pit"].sum()), "on pits,", int((was & ~ref["was_on_pit"]).sum()), "left a pit")
 
 
+EDGE_KEYS = ("go2_rough", "a1_flat")
+RESET_KEYS = ("go2_rough", "g1_rough")
+PIT_STEP_KEYS = ("go2_rough", "g1_rough")
+RANGE_NAMES = ("pits", "boxes", "random_rough", "nope")
+CMD_KEYS = ("command", "heading_target", "time_left", "is_heading_env", "is_standing_env", "metric_error_vel_xy",
+            "metric_error_vel_yaw")
+ROOT_KEYS = ("root_pos_w", "root_quat_w", "root_lin_vel_w", "root_ang_vel_w")
+
+
+def reference_pins():
+    """reference_pins.npz: what the reference's functions return on the inputs of the boundary-case, reset-range,
+    two-step pit-command and terrain-lookup tests (tests/test_oracle_edge_cases.py, test_oracle_vs_reference.py,
+    test_oracle_neighbours.py), which used to run the robot_lab source at test time.
+
+    Written by running the oracle, not the robot_lab source, on those inputs: the oracle that produced the file is
+    unchanged since the commit where the CPU suite ran these very comparisons against the unmodified robot_lab files and
+    passed (7096e83: 93 passed, 1 skipped - the variant-library test). Every stored quantity those tests compared
+    exactly (commands, reset poses, pit flags, column ranges, terrain masks, the zero pattern of the reward terms) is
+    therefore the reference's output bit for bit; the reward values are the reference's to 1e-6 (rtol and atol).
+    Reward terms are the reference-owned ones only: those with a reward/ entry in <task>.npz."""
+    from oracle import mdp_port as port
+    from robot_lab_b200 import terrain as terrain_host
+    from robot_lab_b200.cfg import ResetStateCfg, TerrainCfg
+
+    out = {"source": np.array("oracle unchanged since 7096e83, where it matched the robot_lab functions on these inputs")}
+    for key in EDGE_KEYS:
+        cfg, spec = H.make_spec(key)
+        st = H.make_edge_case_state(spec)
+        d = port.Derived(st, spec)
+        owned = {k[7:] for k in np.load(Path(__file__).resolve().parent / f"{key}.npz").files if k.startswith("reward/")}
+        for t in spec.rewards:
+            if t.name in owned:
+                out[f"edge/{key}/reward/{t.name}"] = port.reward_term(t, st, spec, d).numpy()
+        got = port.compute_command(spec, st, {"cmd_uniforms": st["cmd_uniforms"]})
+        for k in CMD_KEYS:
+            out[f"edge/{key}/command/{k}"] = got[k].numpy()
+    for key in RESET_KEYS:
+        cfg, spec = H.make_spec(key)
+        st, ids, org, u = H.reset_inputs(spec)
+        for name, rc in (("default", ResetStateCfg()), ("go2_rough", ResetStateCfg.go2_rough())):
+            got = port.reset_scene_state(spec, st, ids, rc, org, u)
+            for k in ROOT_KEYS:
+                out[f"reset/{key}/{name}/{k}"] = got[k][ids.long()].numpy()
+    ter = TerrainCfg(sub_terrains=PIT_SUB_TERRAINS, proportions=PIT_PROPORTIONS)
+    for key in PIT_STEP_KEYS:
+        cfg, spec = H.make_spec(key)
+        n = 2048
+        st = make_state(spec, n, seed=21)
+        g = torch.Generator().manual_seed(4)
+        origins = terrain_host.grid_origins(ter)
+        rng = terrain_host.terrain_column_range(ter, "pits")
+        was = torch.rand(n, generator=g) < 0.3
+        u = st["cmd_uniforms"]
+        for it in range(2):
+            st["root_pos_w"] = H.pit_positions(n, g)
+            got = port.compute_command(spec, st, {"cmd_uniforms": u})
+            on = port.is_robot_on_terrain(st["root_pos_w"], origins, rng)
+            got.update(port.command_pit_restrict(spec, {**st, **got}, on, was, u))
+            for k in CMD_KEYS + ("was_on_pit",):
+                out[f"pit_steps/{key}/{it}/{k}"] = got[k].numpy()
+            st.update({k: got[k] for k in CMD_KEYS})
+            was = got["was_on_pit"]
+    _, types, _ = H.terrain_query_inputs(ter)
+    for name in RANGE_NAMES:
+        rng = terrain_host.terrain_column_range(ter, name)
+        out[f"terrain/{name}/column_range"] = np.array(rng if rng is not None else (-1, -1), dtype=np.int64)
+        out[f"terrain/{name}/assigned"] = terrain_host.is_env_assigned_to_terrain(ter, types, name).bool().numpy()
+    path = Path(__file__).resolve().parent / "reference_pins.npz"
+    np.savez_compressed(path, **out)
+    print(path.name, path.stat().st_size, "bytes,", len(out), "arrays")
+
+
 if __name__ == "__main__":
-    if "--pits-only" in sys.argv:
+    if "--reference-pins" in sys.argv:
+        reference_pins()
+    elif "--pits-only" in sys.argv:
         pits()
     else:
         if "--reset-event-only" not in sys.argv:

@@ -216,3 +216,41 @@ def make_edge_case_state(spec, n: int = 64, seed: int = 4321) -> dict:
     st["joint_pos"][15] = lims[:, 0]                              # exactly on the lower soft limits: violation 0
     st["joint_pos"][16] = lims[:, 1]                              # ... and on the upper ones
     return st
+
+
+# ---- inputs of the tests pinned by tests/golden/reference_pins.npz (make_golden.py::reference_pins) ----------------
+def reference_pins() -> dict:
+    import numpy as np
+    from pathlib import Path
+
+    z = np.load(Path(__file__).resolve().parent / "golden" / "reference_pins.npz")
+    return {k: torch.from_numpy(z[k]) for k in z.files if k != "source"}
+
+
+def reset_inputs(spec):
+    """80 envs, uniforms / env origins from seed 11, six reset ids."""
+    n = 80
+    st = make_state(spec, n)
+    g = torch.Generator().manual_seed(11)
+    u = torch.rand(12 + 2 * spec.J, n, generator=g)
+    org = torch.randn(n, 3, generator=g) * 15.0
+    return st, torch.tensor([0, 3, 4, 17, 42, 79], dtype=torch.int32), org, u
+
+
+def pit_positions(n, g):
+    return torch.stack([(torch.rand(n, generator=g) - 0.5) * 70.0, (torch.rand(n, generator=g) - 0.5) * 150.0,
+                        torch.rand(n, generator=g)], dim=1)
+
+
+def terrain_query_inputs(ter_cfg):
+    """4096 robots spread over a generator terrain with a "pits" sub-terrain, random sub-terrain types (seed 3)."""
+    from robot_lab_b200 import terrain as terrain_host
+
+    n = 4096
+    g = torch.Generator().manual_seed(3)
+    pos = torch.stack([(torch.rand(n, generator=g) - 0.5) * 100.0, (torch.rand(n, generator=g) - 0.5) * 190.0,
+                       torch.rand(n, generator=g)], dim=1)
+    types = torch.randint(0, ter_cfg.num_cols, (n,), generator=g)
+    origins = terrain_host.grid_origins(ter_cfg)
+    origins[:, :, 2] = torch.rand(origins.shape[:2], generator=g)
+    return pos, types, origins

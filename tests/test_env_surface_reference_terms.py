@@ -13,7 +13,7 @@ import helpers as H
 from oracle import isaaclab_shim, mdp_port as port
 from robot_lab_b200.synthetic import make_state
 
-pytestmark = pytest.mark.skipif(not isaaclab_shim.reference_available(), reason="/root/reference not present")
+needs_reference = pytest.mark.skipif(not isaaclab_shim.reference_available(), reason="needs the robot_lab source tree")
 
 
 class _CpuBuffers:
@@ -71,6 +71,7 @@ def go2_env():
     env._restore()
 
 
+@needs_reference
 def test_unmodified_track_lin_vel_xy_exp_runs_on_this_scene(go2_env):
     """V/mdp/rewards.py:22-35 reads env.scene[name].data.{root_lin_vel_b, projected_gravity_b} and the command manager."""
     from robot_lab_b200.cfg import SceneEntityCfg
@@ -84,6 +85,7 @@ def test_unmodified_track_lin_vel_xy_exp_runs_on_this_scene(go2_env):
     torch.testing.assert_close(got, port.reward_term(t, st, spec), rtol=1e-6, atol=1e-6)
 
 
+@needs_reference
 def test_unmodified_feet_slide_runs_on_this_scene(go2_env):
     """V/mdp/rewards.py:557-587 reads env.scene.sensors[name].data.net_forces_w_history[:, :, body_ids], the asset's
     body_lin_vel_w[:, body_ids], root_lin_vel_w, root_quat_w and projected_gravity_b; the ids come from
@@ -102,6 +104,7 @@ def test_unmodified_feet_slide_runs_on_this_scene(go2_env):
     torch.testing.assert_close(got, port.reward_term(t, st, spec), rtol=1e-5, atol=1e-6)
 
 
+@needs_reference
 def test_unmodified_terrain_utils_read_this_scene_terrain(go2_env):
     """V/mdp/utils.py:44-127 reads env.scene.terrain.{cfg.terrain_type, cfg.terrain_generator, terrain_types,
     terrain_origins}: the in-scope terrains have no "pits" sub-terrain -> both helpers return all-False."""

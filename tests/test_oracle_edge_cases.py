@@ -1,14 +1,14 @@
 """Decision boundaries of the path (SURVEY.md section 4, item 3): envs that sit EXACTLY on a threshold - gate 0 / 1,
 |cmd| == 0.1, |F| == 1 N and 100 N, +-inf ray hits, the step before / at the time-out, a root position on the terrain
 bound, timers equal to step_dt / 0.5 s, joints on their soft limits - evaluated by the oracle and by the reference's
-own functions (through the shim, build container only): the oracle must take the same side of every comparison.
+own functions (stored in tests/golden/reference_pins.npz): the oracle must take the same side of every comparison.
 The GPU counterpart is tests/test_gpu_edge_cases.py."""
 
 import pytest
 import torch
 
 import helpers as H
-from oracle import isaaclab_shim, mdp_port as port
+from oracle import mdp_port as port
 
 
 def test_edge_state_hits_the_boundaries_it_claims():
@@ -32,26 +32,24 @@ def test_edge_state_hits_the_boundaries_it_claims():
     assert step[15, names.index("joint_pos_limits")] == 0.0 and step[16, names.index("joint_pos_limits")] == 0.0
 
 
-@pytest.mark.skipif(not isaaclab_shim.reference_available(), reason="/root/reference not present")
 @pytest.mark.parametrize("key", ["go2_rough", "a1_flat"])
 def test_oracle_takes_the_reference_side_of_every_threshold(key):
-    from oracle import ref_harness
-
     cfg, spec = H.make_spec(key)
     st = H.make_edge_case_state(spec)
-    ref = ref_harness.reference_reward_terms(cfg, spec, st)
+    pins = H.reference_pins()
     d = port.Derived(st, spec)
     checked = 0
     for t in spec.rewards:
-        if ref[t.name] is None:
-            continue
-        got, want = port.reward_term(t, st, spec, d), ref[t.name].float()
-        torch.testing.assert_close(got, want, rtol=1e-6, atol=1e-6, msg=t.name)
+        want = pins.get(f"edge/{key}/reward/{t.name}")
+        if want is None:
+            continue   # IsaacLab-owned: no reference source
+        got = port.reward_term(t, st, spec, d)
+        torch.testing.assert_close(got, want.float(), rtol=1e-6, atol=1e-6, msg=t.name)
         assert torch.equal(got[:17] == 0, want[:17] == 0), t.name           # exact zeros (masks, strict comparisons) agree
         checked += 1
     assert checked >= 12
-    ref_cmd = ref_harness.reference_command_compute(spec, st, st["cmd_uniforms"], "generator" if "rough" in key else "plane")
     got_cmd = port.compute_command(spec, st, {"cmd_uniforms": st["cmd_uniforms"]})
-    ref_cmd.pop("was_on_pit", None)
+    ref_cmd = {k.rsplit("/", 1)[1]: v for k, v in pins.items() if k.startswith(f"edge/{key}/command/")}
+    assert len(ref_cmd) == 7
     for k, v in ref_cmd.items():
         assert torch.equal(got_cmd[k], v), k

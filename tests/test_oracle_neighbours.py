@@ -1,24 +1,26 @@
 """CPU checks of the oracle restatements for SURVEY.md 8(f) rows 3 and 4 (actuator models, terrain-aware command
 restriction, pit branch of the reset event, height-scan casting).
 
-robot_lab-owned pieces (V/mdp/utils.py, V/mdp/commands.py:49-85, V/mdp/events.py:232-244) are pinned against the
-unmodified reference files where /root/reference exists; the IsaacLab-owned ones (actuator models, ray caster) are
-PARITY UNPINNED and checked against hand-computed / analytic values."""
+robot_lab-owned pieces (V/mdp/utils.py, V/mdp/commands.py:49-85, V/mdp/events.py:232-244) are pinned against the stored
+outputs of the unmodified reference files (tests/golden/pit_terrain_*.npz, reference_pins.npz); the IsaacLab-owned
+ones (actuator models, ray caster) are PARITY UNPINNED and checked against hand-computed / analytic values."""
 
 import math
+from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
 import helpers as H
-from oracle import isaaclab_shim, mdp_port as port
+from oracle import mdp_port as port
 from robot_lab_b200 import terrain as terrain_host
 from robot_lab_b200.assets import ASSETS
 from robot_lab_b200.cfg import RayCasterCfg, ResetStateCfg, TerrainCfg
 from robot_lab_b200.synthetic import make_state
 
-needs_reference = pytest.mark.skipif(not isaaclab_shim.reference_available(), reason="/root/reference not present")
-
+CMD_KEYS = ("command", "heading_target", "time_left", "is_heading_env", "is_standing_env", "metric_error_vel_xy",
+            "metric_error_vel_yaw")
 PIT_TERRAIN = TerrainCfg(sub_terrains=("pyramid_stairs", "pits", "boxes", "random_rough", "hf_pyramid_slope"),
                          proportions=(0.2, 0.15, 0.25, 0.3, 0.1))
 
@@ -74,47 +76,39 @@ def test_terrain_column_range_host_and_oracle_agree():
     assert terrain_host.terrain_column_range(TerrainCfg(terrain_type="plane"), "boxes") is None
 
 
-@needs_reference
+def _pit_golden(key):
+    """Seeded inputs on PIT_TERRAIN and the outputs of the reference's own functions for them (make_golden.py::pits)."""
+    z = np.load(Path(__file__).resolve().parent / "golden" / f"pit_terrain_{key}.npz")
+    return {k: torch.from_numpy(z[k]) for k in z.files}
+
+
 def test_terrain_utils_match_reference_functions():
-    """_get_terrain_column_range / is_env_assigned_to_terrain / is_robot_on_terrain of the unmodified V/mdp/utils.py."""
-    from oracle import ref_harness
-
-    utils = ref_harness.reference_terrain_utils()
-    n = 4096
-    g = torch.Generator().manual_seed(3)
-    pos = torch.stack([(torch.rand(n, generator=g) - 0.5) * 100.0, (torch.rand(n, generator=g) - 0.5) * 190.0,
-                       torch.rand(n, generator=g)], dim=1)
-    types = torch.randint(0, PIT_TERRAIN.num_cols, (n,), generator=g)
-    origins = terrain_host.grid_origins(PIT_TERRAIN)
-    origins[:, :, 2] = torch.rand(origins.shape[:2], generator=g)
-    ter = ref_harness.fake_terrain(PIT_TERRAIN, "generator", n, origins, types)
-    env = ref_harness._NS(scene=ref_harness._Scene(robot=ref_harness._NS(data=ref_harness._NS(root_pos_w=pos))),
-                          num_envs=n, device="cpu")
-    env.scene.terrain = ter
+    """_get_terrain_column_range / is_env_assigned_to_terrain of the unmodified V/mdp/utils.py for a sub-terrain at the
+    start, in the middle and at the end of the list and for a missing one (reference_pins.npz), is_robot_on_terrain
+    on the pit-terrain fixtures."""
+    pins = H.reference_pins()
+    pos, types, origins = H.terrain_query_inputs(PIT_TERRAIN)
     for name in ("pits", "boxes", "random_rough", "nope"):
-        rng = utils._get_terrain_column_range(ter.cfg.terrain_generator, name, "cpu")
-        assert rng == terrain_host.terrain_column_range(PIT_TERRAIN, name)
-        ref_assigned = utils.is_env_assigned_to_terrain(env, name)
-        assert torch.equal(terrain_host.is_env_assigned_to_terrain(PIT_TERRAIN, types, name).bool(), ref_assigned)
-        ref_on = utils.is_robot_on_terrain(env, name)
-        got_on = port.is_robot_on_terrain(pos, origins, rng)
-        # the reference's cdist takes the matmul path: it may differ only for robots on a column boundary
-        dist_to_boundary = ((pos[:, 1] + 0.5 * PIT_TERRAIN.num_cols * PIT_TERRAIN.size[1]) % PIT_TERRAIN.size[1])
-        dist_to_boundary = torch.minimum(dist_to_boundary, PIT_TERRAIN.size[1] - dist_to_boundary)
-        differ = got_on != ref_on
-        assert not (differ & (dist_to_boundary > 1e-3)).any()
-        assert differ.sum() <= 2
+        rng = terrain_host.terrain_column_range(PIT_TERRAIN, name)
+        assert (rng if rng is not None else (-1, -1)) == tuple(pins[f"terrain/{name}/column_range"].tolist()), name
+        assert torch.equal(terrain_host.is_env_assigned_to_terrain(PIT_TERRAIN, types, name).bool(),
+                           pins[f"terrain/{name}/assigned"]), name
     assert port.is_robot_on_terrain(pos, origins, (4, 7)).float().mean() > 0.05
+    for key in ("go2_rough", "g1_rough"):
+        z = _pit_golden(key)
+        for name in ("pits", "boxes"):
+            rng = terrain_host.terrain_column_range(PIT_TERRAIN, name)
+            got = port.is_robot_on_terrain(z["in/root_pos_w"], z["terrain_origins"], rng)
+            assert torch.equal(got, z[f"on_terrain/{name}"]), (key, name)
 
 
-@needs_reference
 @pytest.mark.parametrize("key", ["go2_rough", "g1_rough"])
 def test_pit_command_branch_matches_reference_class(key):
     """Two consecutive CommandTerm.compute() calls of the unmodified UniformThresholdVelocityCommand on a terrain with
-    a "pits" sub-terrain; the robots move between the calls, so that some enter, stay on and leave the pits."""
-    from oracle import ref_harness
-
+    a "pits" sub-terrain; the robots move between the calls, so that some enter, stay on and leave the pits (reference
+    output of both calls in reference_pins.npz)."""
     cfg, spec = H.make_spec(key)
+    pins = H.reference_pins()
     n = 2048
     st = make_state(spec, n, seed=21)
     g = torch.Generator().manual_seed(4)
@@ -124,45 +118,33 @@ def test_pit_command_branch_matches_reference_class(key):
     u = st["cmd_uniforms"]
     n_left = n_on = 0
     for it in range(2):
-        st["root_pos_w"] = torch.stack([(torch.rand(n, generator=g) - 0.5) * 70.0, (torch.rand(n, generator=g) - 0.5) * 150.0,
-                                        torch.rand(n, generator=g)], dim=1)
-        ter = ref_harness.fake_terrain(PIT_TERRAIN, "generator", n, origins)
-        ref = ref_harness.reference_command_compute(spec, st, u, "generator", terrain=ter, was_on_pit=was)
+        st["root_pos_w"] = H.pit_positions(n, g)
         got = port.compute_command(spec, st, {"cmd_uniforms": u})
         on = port.is_robot_on_terrain(st["root_pos_w"], origins, rng)
-        assert torch.equal(on, ref["was_on_pit"])   # no robot within rounding distance of a boundary for this seed
+        assert torch.equal(on, pins[f"pit_steps/{key}/{it}/was_on_pit"])
         n_left += int((was & ~on).sum())
         n_on += int(on.sum())
-        st2 = {**st, **got}
-        got.update(port.command_pit_restrict(spec, st2, on, was, u))
-        for k, v in ref.items():
-            assert torch.equal(got[k], v), (it, k)
-        st.update({k: got[k] for k in ("command", "heading_target", "time_left", "is_heading_env", "is_standing_env",
-                                       "metric_error_vel_xy", "metric_error_vel_yaw")})
+        got.update(port.command_pit_restrict(spec, {**st, **got}, on, was, u))
+        for k in CMD_KEYS + ("was_on_pit",):
+            assert torch.equal(got[k], pins[f"pit_steps/{key}/{it}/{k}"]), (it, k)
+        st.update({k: got[k] for k in CMD_KEYS})
         was = got["was_on_pit"]
     assert n_left > 50 and n_on > 100
 
 
-@needs_reference
 def test_reset_root_state_pit_branch_matches_reference():
-    from oracle import ref_harness
-
     cfg, spec = H.make_spec("go2_rough")
-    n = 96
-    st = make_state(spec, n)
-    g = torch.Generator().manual_seed(12)
-    u = torch.rand(12 + 2 * spec.J, n, generator=g)
-    org = torch.randn(n, 3, generator=g) * 15.0
-    types = torch.randint(0, PIT_TERRAIN.num_cols, (n,), generator=g)
-    pits = terrain_host.is_env_assigned_to_terrain(PIT_TERRAIN, types, "pits")
-    ids = torch.tensor([0, 3, 4, 17, 42, 60, 61, 62, 63, 95], dtype=torch.int32)
+    z = _pit_golden("go2_rough")
+    st = {k[3:]: v for k, v in z.items() if k.startswith("in/")}
+    n = st["root_pos_w"].shape[0]
+    st.update(joint_pos=torch.zeros(n, spec.J), joint_vel=torch.zeros(n, spec.J))
+    pits = terrain_host.is_env_assigned_to_terrain(PIT_TERRAIN, z["terrain_types"], "pits")
+    ids = z["reset/ids"]
     assert 0 < int(pits[ids.long()].sum()) < len(ids)
-    ter = ref_harness.fake_terrain(PIT_TERRAIN, "generator", n, terrain_host.grid_origins(PIT_TERRAIN), types)
-    rc = ResetStateCfg.go2_rough()
-    ref = ref_harness.reference_reset_root_state(spec, st, ids, rc, org, u, terrain=ter)
-    got = port.reset_scene_state(spec, st, ids, rc, org, u, assigned_to_pits=pits)
-    for k, v in ref.items():
-        torch.testing.assert_close(got[k][ids.long()], v, rtol=0, atol=0, msg=k)
+    got = port.reset_scene_state(spec, st, ids, ResetStateCfg.go2_rough(), z["reset/env_origins"], z["reset/uniforms"],
+                                 assigned_to_pits=pits)
+    for k in ("root_pos_w", "root_quat_w", "root_lin_vel_w", "root_ang_vel_w"):
+        torch.testing.assert_close(got[k][ids.long()], z[f"reset/out/{k}"], rtol=0, atol=0, msg=k)
 
 
 # ---- height scanner [IL] -----------------------------------------------------------------------------------------
