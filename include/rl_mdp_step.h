@@ -27,6 +27,8 @@
  *                              (V/mdp/commands.py:61-85)
  *   rl_height_scan_cast        the grid-pattern RayCaster [IL] (V/velocity_env_cfg.py:70-77) over a height-field
  *                              terrain: produces ray_hits_z / ray_sensor_pos_z for the height_scan observation
+ *   rl_interval_push           EventManager.reset / apply("interval") [IL] for one non-global interval term running
+ *                              push_by_setting_velocity [IL] (randomize_push_robot, V/velocity_env_cfg.py:366-371)
  *
  * Conventions: every function returns 0 on success or a negative RL_E* code; rl_last_error() gives the
  * message (thread-local). All data pointers are DEVICE pointers borrowed for the duration of the call;
@@ -43,7 +45,7 @@
 extern "C" {
 #endif
 
-#define RL_ABI_VERSION 12
+#define RL_ABI_VERSION 13
 
 #define RL_MAX_JOINTS 64
 #define RL_MAX_BODIES 64        /* bodies in the contact-force history tensor                  */
@@ -57,6 +59,7 @@ extern "C" {
 #define RL_DEBUG_STRIDE 160     /* int64 words per CTA in the debug buffer */
 #define RL_NUM_OBS_GROUPS 2     /* 0 = policy, 1 = critic                                        */
 #define RL_NUM_CMD_UNIFORMS 7   /* time_left, vx, vy, wz, heading, is_heading, is_standing       */
+#define RL_NUM_INTERVAL_UNIFORMS 8 /* rl_interval_push: timer on reset, timer on fire, 6 velocities */
 
 enum RlError {
   RL_OK = 0,
@@ -566,6 +569,40 @@ typedef struct RlHeightField {
 
 int rl_height_scan_cast(RlCtx* ctx, int64_t num_envs, const RlHeightField* hf, const RlStateView* state /* reads
                         root_pos_w, root_quat_w; writes ray_hits_z, ray_sensor_pos_z */, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Stage 8 of ManagerBasedRLEnv.step() [IL]: event_manager.apply("interval", dt=step_dt) for one non-global interval
+ * term (EventTermCfg(mode="interval", is_global_time=False)) whose function is push_by_setting_velocity [IL]; the
+ * reference's randomize_push_robot (V/velocity_env_cfg.py:366-371). IsaacLab semantics (isaaclab/managers/
+ * event_manager.py, isaaclab/envs/mdp/events.py), with sample_uniform(lo, hi) = u * (hi - lo) + lo, u in [0, 1):
+ *   construction / EventManager.reset(ids):  time_left[ids] = sample_uniform(interval_lo, interval_hi)
+ *   apply("interval", dt):                   time_left -= dt
+ *                                            fire = time_left < 1e-6
+ *                                            time_left[fire] = sample_uniform(interval_lo, interval_hi)
+ *                                            root_vel_w[fire] += sample_uniform(vel_lo, vel_hi)   (6 components)
+ * root_vel_w is (root_lin_vel_w x, y, z, root_ang_vel_w x, y, z); body velocities are not touched.
+ */
+typedef struct RlIntervalEventCfg {
+  float interval_lo, interval_hi;     /* EventTermCfg.interval_range_s                                       */
+  float vel_lo[6], vel_hi[6];         /* velocity_range x, y, z, roll, pitch, yaw; a missing key is (0, 0)   */
+} RlIntervalEventCfg;
+
+/* Two forms:
+ *   reset form (env_ids != NULL): time_left[env_ids[0 .. *n_env_ids)] resampled; nothing else is read or written
+ *     (pushed_ids / n_pushed may be NULL).
+ *   step form (env_ids == NULL): one thread per env; an env whose terminated | truncated byte is set first gets a fresh
+ *     timer (the reset of stage 6 of the step), then every env is decremented, compared and pushed. The ids of the
+ *     pushed envs are written to pushed_ids[0 .. *n_pushed) in no particular order; *n_pushed is zeroed on the stream
+ *     by the call itself, so it is defined after every launch without a host round trip (a CUDA graph replays it).
+ *     A simulator writes the root velocities of exactly those envs back (write_root_velocity_to_sim [IL]).
+ * time_left is a DEVICE float [N]; state->root_lin_vel_w / root_ang_vel_w are read and written.
+ * Uniforms: Philox streams RL_STREAM_INTERVAL_RESET (timer on reset) / RL_STREAM_INTERVAL_PUSH (timer on fire, six
+ * velocity components) of `rnd`, or `uniforms` = [8][N] U[0,1) when not NULL: row 0 timer on reset, row 1 timer on fire,
+ * rows 2-7 velocity x, y, z, roll, pitch, yaw. */
+int rl_interval_push(RlCtx* ctx, int64_t num_envs, const RlIntervalEventCfg* cfg, float dt, float* time_left,
+                     const RlStateView* state, const uint8_t* terminated, const uint8_t* truncated,
+                     const int32_t* env_ids, const int32_t* n_env_ids, int32_t* pushed_ids /* [N] */,
+                     int32_t* n_pushed /* device [1] */, const RlRandom* rnd, const float* uniforms, void* stream);
 
 /* The fused step over envs [0, num_envs), or over env_ids[0 .. *n_env_ids) when env_ids != NULL
  * (n_env_ids is a DEVICE pointer so that no host sync is needed after the reset compaction). */

@@ -14,7 +14,7 @@ from pathlib import Path
 
 import torch
 
-RL_ABI_VERSION = 12
+RL_ABI_VERSION = 13
 RL_MAX_TASKS = 112
 RL_DEBUG_STRIDE = 160
 RL_MAX_JOINTS = 64
@@ -181,6 +181,14 @@ class RlHeightField(C.Structure):
                 ("ray_starts", C.c_void_p)]
 
 
+class RlIntervalEventCfg(C.Structure):
+    _fields_ = [("interval_lo", C.c_float), ("interval_hi", C.c_float), ("vel_lo", C.c_float * 6), ("vel_hi", C.c_float * 6)]
+
+
+# rows of the uniform table of rl_interval_push ([8][N]): timer on reset, timer on fire, velocity x, y, z, roll, pitch, yaw
+RL_NUM_INTERVAL_UNIFORMS = 8
+
+
 class RlStepOut(C.Structure):
     _fields_ = [
         ("obs", C.c_void_p * RL_NUM_OBS_GROUPS), ("obs_pitch", C.c_int64 * RL_NUM_OBS_GROUPS),
@@ -198,13 +206,14 @@ class RlRandom(C.Structure):
 
 _STRUCTS = (RlRewardTerm, RlObsTerm, RlObsGroup, RlDoneTerm, RlCommandCfg, RlActionCfg, RlStepSpec, RlField,
             RlStateView, RlMdpState, RlStepOut, RlRandom, RlResetLog, RlResetStateCfg, RlActuatorCfg, RlTerrainGrid,
-            RlHeightField)
+            RlHeightField, RlIntervalEventCfg)
 
 EXPORTED_SYMBOLS = (
     "rl_abi_version", "rl_last_error", "rl_struct_sizeof", "rl_tile_record_bytes", "rl_ctx_create", "rl_ctx_destroy",
     "rl_ctx_set_launch_config", "rl_ctx_get_launch_config", "rl_ctx_get_cluster_config", "rl_ctx_set_pdl", "rl_ctx_set_debug_buffer", "rl_ctx_get_schedule",
     "rl_contact_sensor_update", "rl_reset_scene_state", "rl_process_action", "rl_step", "rl_reset_envs", "rl_term_eval",
     "rl_actuator_step", "rl_is_robot_on_terrain", "rl_command_pit_restrict", "rl_height_scan_cast", "rl_derived_views",
+    "rl_interval_push",
 )
 
 LIB_PATH = Path(__file__).resolve().parent / "_lib" / "libmdpstep.so"
@@ -265,6 +274,9 @@ def load() -> C.CDLL:
                                         C.c_void_p]
     lib.rl_derived_views.argtypes = [C.c_void_p, C.c_int64, C.POINTER(RlStateView), C.POINTER(RlField), C.POINTER(RlField),
                                      C.POINTER(RlField), C.POINTER(RlField), C.c_void_p]
+    lib.rl_interval_push.argtypes = [C.c_void_p, C.c_int64, C.POINTER(RlIntervalEventCfg), C.c_float, C.c_void_p,
+                                     C.POINTER(RlStateView), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.POINTER(RlRandom), C.c_void_p, C.c_void_p]
     lib.rl_contact_sensor_update.argtypes = [C.c_void_p, C.c_int64, C.POINTER(RlField), C.POINTER(RlStateView),
                                              C.POINTER(C.c_int32), C.c_float, C.c_float, C.c_int32, C.c_void_p]
     lib.rl_process_action.argtypes = [C.c_void_p, C.c_int64, C.POINTER(RlField), C.POINTER(RlMdpState),

@@ -134,6 +134,18 @@ class TerminationTermCfg:
     time_out: bool = False
 
 
+@dataclass
+class EventTermCfg:
+    """EventTermCfg [IL] (isaaclab.managers.EventTermCfg): ``func`` applied in ``mode`` ("startup" | "reset" |
+    "interval"); interval terms fire every ``interval_range_s`` seconds, drawn per env unless ``is_global_time``."""
+
+    func: Callable
+    mode: str
+    interval_range_s: tuple[float, float] | None = None
+    is_global_time: bool = False
+    params: dict[str, Any] = field(default_factory=dict)
+
+
 class TermContainer:
     """An ordered bag of named terms; attribute order = insertion order (the managers iterate in it).
 

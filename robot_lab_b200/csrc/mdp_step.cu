@@ -1036,7 +1036,7 @@ int64_t rl_struct_sizeof(const char* name) {
   RL_SZ(RlRewardTerm); RL_SZ(RlObsTerm); RL_SZ(RlObsGroup); RL_SZ(RlDoneTerm); RL_SZ(RlCommandCfg);
   RL_SZ(RlActionCfg); RL_SZ(RlStepSpec); RL_SZ(RlField); RL_SZ(RlStateView); RL_SZ(RlMdpState);
   RL_SZ(RlStepOut); RL_SZ(RlRandom); RL_SZ(RlResetLog); RL_SZ(RlResetStateCfg);
-  RL_SZ(RlActuatorCfg); RL_SZ(RlTerrainGrid); RL_SZ(RlHeightField);
+  RL_SZ(RlActuatorCfg); RL_SZ(RlTerrainGrid); RL_SZ(RlHeightField); RL_SZ(RlIntervalEventCfg);
 #undef RL_SZ
   return -1;
 }

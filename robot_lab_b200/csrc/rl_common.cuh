@@ -49,7 +49,7 @@ const RlStepSpec* rl_ctx_spec_of(const RlCtx* ctx);
 // ---------------------------------------------------------------------------------------------------
 enum {
   RL_STREAM_COMMAND = 1, RL_STREAM_RESET_COMMAND = 2, RL_STREAM_RESET_STATE = 3, RL_STREAM_RESET_JOINTS = 4,
-  RL_STREAM_PIT_RESAMPLE = 5, RL_STREAM_OBS = 16
+  RL_STREAM_PIT_RESAMPLE = 5, RL_STREAM_INTERVAL_RESET = 6, RL_STREAM_INTERVAL_PUSH = 7, RL_STREAM_OBS = 16
 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
@@ -78,6 +78,16 @@ __device__ __forceinline__ RandState rl_rand_state(const RlRandom& rnd) {
   return rs;
 }
 static __device__ __noinline__ uint4 rl_philox(const RandState r, long long env, uint32_t stream, uint32_t block) {
+  const unsigned long long genv = (unsigned long long)(env + r.env_id_offset);
+  uint4 ctr = make_uint4((uint32_t)genv, (uint32_t)r.step, (uint32_t)(r.step >> 32) ^ (uint32_t)(genv >> 32),
+                         (stream << 16) | block);
+  return philox4x32_10(ctr, make_uint2((uint32_t)r.seed, (uint32_t)(r.seed >> 32)));
+}
+
+// The same draw as rl_philox, inlined into its caller. For kernels added to a translation unit whose existing kernels
+// call rl_philox: a new call site of the out-of-line copy changes how the compiler fits that copy (and the code of its
+// existing callers) to its call sites.
+__device__ __forceinline__ uint4 rl_philox_inline(const RandState r, long long env, uint32_t stream, uint32_t block) {
   const unsigned long long genv = (unsigned long long)(env + r.env_id_offset);
   uint4 ctr = make_uint4((uint32_t)genv, (uint32_t)r.step, (uint32_t)(r.step >> 32) ^ (uint32_t)(genv >> 32),
                          (stream << 16) | block);

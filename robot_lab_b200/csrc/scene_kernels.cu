@@ -6,8 +6,10 @@
 //   rl_is_robot_on_terrain   is_robot_on_terrain (V/mdp/utils.py:73-127)
 //   rl_command_pit_restrict  tail of UniformThresholdVelocityCommand._update_command (V/mdp/commands.py:61-85)
 //   rl_height_scan_cast      grid-pattern RayCaster [IL] (V/velocity_env_cfg.py:70-77) over a height-field terrain
+//   rl_interval_push         EventManager.reset / apply("interval") [IL] with push_by_setting_velocity [IL]
+//                            (randomize_push_robot, V/velocity_env_cfg.py:366-371)
 //
-// All four are per-env maps over a few hundred bytes per env: HBM / L2 bound elementwise work, no tensor cores.
+// All of them are per-env maps over a few hundred bytes per env: HBM / L2 bound elementwise work, no tensor cores.
 // Index order follows the layout of the tensor being written so that SoA [C][N] and IsaacLab-shaped AoS [N][C]
 // tensors both coalesce. Built with -fmad=false like mdp_step.cu: the reference is eager PyTorch, every op rounds.
 
@@ -283,6 +285,88 @@ __global__ void __launch_bounds__(256) derived_views_kernel(const __grid_constan
   }
 }
 
+// ---------------------------------------------------------------------------------------------------
+// Interval push event [IL]: EventManager._prepare_terms / reset / apply("interval") for one non-global interval term
+// (isaaclab/managers/event_manager.py) and its function push_by_setting_velocity (isaaclab/envs/mdp/events.py). One
+// thread per env (step form) or per listed id (reset form): a few bytes per env, no reuse. The pushed ids leave through
+// one atomic per warp (ballot + prefix popcount), so their order within the list is unspecified.
+// ---------------------------------------------------------------------------------------------------
+struct IntervalArgs {
+  int N;
+  float dt;
+  RlIntervalEventCfg cfg;
+  float* time_left;
+  RlField lin, ang;
+  const uint8_t* terminated;
+  const uint8_t* truncated;
+  const int32_t* env_ids;
+  const int32_t* n_env_ids;
+  int32_t* pushed_ids;
+  int32_t* n_pushed;
+  RlRandom rnd;
+  const float* uniforms;   // [8][N] or NULL: timer on reset, timer on fire, velocity x, y, z, roll, pitch, yaw
+};
+
+// torch.rand(n) * (upper - lower) + lower [IL], the interval sample of _prepare_terms, reset and apply
+__device__ __forceinline__ float interval_sample(const RlIntervalEventCfg& c, float u) {
+  return u * (c.interval_hi - c.interval_lo) + c.interval_lo;
+}
+
+__device__ __forceinline__ float interval_reset_uniform(const IntervalArgs& a, long long env) {
+  if (a.uniforms) return a.uniforms[env];
+  return u01(rl_philox_inline(rl_rand_state(a.rnd), env, RL_STREAM_INTERVAL_RESET, 0).x);
+}
+
+__global__ void __launch_bounds__(256) interval_reset_kernel(const __grid_constant__ IntervalArgs a) {
+  const int n = *a.n_env_ids;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const long long env = a.env_ids[i];
+    a.time_left[env] = interval_sample(a.cfg, interval_reset_uniform(a, env));
+  }
+}
+
+__global__ void __launch_bounds__(256) interval_step_kernel(const __grid_constant__ IntervalArgs a) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  bool fire = false;
+  if (env < a.N) {
+    float t = a.time_left[env];
+    // EventManager.reset(env_ids) [IL] of the envs reset at stage 6 of this step
+    if ((a.terminated && a.terminated[env]) || (a.truncated && a.truncated[env])) t = interval_sample(a.cfg, interval_reset_uniform(a, env));
+    // apply("interval"): time_left -= dt; time_left < 1e-6 (fp32 tensor against a python scalar: compared in fp32)
+    t = t - a.dt;
+    fire = t < 1e-6f;
+    if (fire) {
+      float u[7];
+      if (a.uniforms) {
+#pragma unroll
+        for (int q = 0; q < 7; ++q) u[q] = a.uniforms[(long long)(q + 1) * a.N + env];
+      } else {
+        const RandState rs = rl_rand_state(a.rnd);
+        const uint4 r0 = rl_philox_inline(rs, env, RL_STREAM_INTERVAL_PUSH, 0), r1 = rl_philox_inline(rs, env, RL_STREAM_INTERVAL_PUSH, 1);
+        u[0] = u01(r0.x); u[1] = u01(r0.y); u[2] = u01(r0.z); u[3] = u01(r0.w);
+        u[4] = u01(r1.x); u[5] = u01(r1.y); u[6] = u01(r1.z);
+      }
+      t = interval_sample(a.cfg, u[0]);
+      // push_by_setting_velocity [IL]: root_vel_w += sample_uniform(ranges[:, 0], ranges[:, 1]) = rand * (hi - lo) + lo
+      const RlIntervalEventCfg& c = a.cfg;
+#pragma unroll
+      for (int q = 0; q < 3; ++q) {
+        st_f(a.lin, env, q, ld_f(a.lin, env, q) + (u[1 + q] * (c.vel_hi[q] - c.vel_lo[q]) + c.vel_lo[q]));
+        st_f(a.ang, env, q, ld_f(a.ang, env, q) + (u[4 + q] * (c.vel_hi[3 + q] - c.vel_lo[3 + q]) + c.vel_lo[3 + q]));
+      }
+    }
+    a.time_left[env] = t;
+  }
+  const unsigned m = __ballot_sync(0xffffffffu, fire);   // whole warps reach this point (no early exit above)
+  if (m) {
+    const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+    int base = 0;
+    if (lane == leader) base = atomicAdd(a.n_pushed, __popc(m));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (fire) a.pushed_ids[base + __popc(m & ((1u << lane) - 1u))] = env;
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -416,6 +500,46 @@ int rl_derived_views(RlCtx* ctx, int64_t num_envs, const RlStateView* state, con
   const int threads = 256;
   const int blocks = (int)((num_envs + threads - 1) / threads);
   derived_views_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  return RL_OK;
+}
+
+int rl_interval_push(RlCtx* ctx, int64_t num_envs, const RlIntervalEventCfg* cfg, float dt, float* time_left,
+                     const RlStateView* state, const uint8_t* terminated, const uint8_t* truncated,
+                     const int32_t* env_ids, const int32_t* n_env_ids, int32_t* pushed_ids, int32_t* n_pushed,
+                     const RlRandom* rnd, const float* uniforms, void* stream) {
+  if (!ctx || !cfg || !time_left || !rnd) return rl_fail(RL_EINVAL, "rl_interval_push: null argument%s", "");
+  if (!(cfg->interval_lo <= cfg->interval_hi))
+    return rl_fail(RL_EINVAL, "rl_interval_push: interval_range_s needs lo <= hi%s", "");
+  for (int q = 0; q < 6; ++q)
+    if (!(cfg->vel_lo[q] <= cfg->vel_hi[q]))
+      return rl_fail(RL_EINVAL, "rl_interval_push: velocity_range component %s%lld needs lo <= hi", "", q);
+  if (num_envs >= (1ll << 31)) return rl_fail(RL_EINVAL, "rl_interval_push: num_envs must stay below 2^31%s", "");
+  IntervalArgs a;
+  memset(&a, 0, sizeof(a));
+  a.N = (int)(num_envs > 0 ? num_envs : 0); a.dt = dt; a.cfg = *cfg; a.time_left = time_left;
+  a.rnd = *rnd; a.uniforms = uniforms;
+  RlDeviceGuard guard(rl_ctx_device_of(ctx));
+  const int threads = 256;
+  const int blocks = (int)((num_envs + threads - 1) / threads);
+  if (env_ids || n_env_ids) {   // reset form
+    if (!env_ids || !n_env_ids) return rl_fail(RL_EINVAL, "rl_interval_push: env_ids and n_env_ids go together%s", "");
+    if (num_envs <= 0) return RL_OK;
+    a.env_ids = env_ids; a.n_env_ids = n_env_ids;
+    interval_reset_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    return RL_OK;
+  }
+  if (!state || !state->root_lin_vel_w.ptr || !state->root_ang_vel_w.ptr)
+    return rl_fail(RL_EINVAL, "rl_interval_push: root_lin_vel_w and root_ang_vel_w are required%s", "");
+  if (!terminated && !truncated) return rl_fail(RL_EINVAL, "rl_interval_push: env_ids or the done masks are required%s", "");
+  if (!pushed_ids || !n_pushed) return rl_fail(RL_EINVAL, "rl_interval_push: pushed_ids and n_pushed are required%s", "");
+  if (!(dt > 0.f)) return rl_fail(RL_EINVAL, "rl_interval_push: dt must be positive%s", "");
+  CUDA_TRY(cudaMemsetAsync(n_pushed, 0, sizeof(int32_t), (cudaStream_t)stream));   // a graph node: defined on every replay
+  if (num_envs <= 0) return RL_OK;
+  a.lin = state->root_lin_vel_w; a.ang = state->root_ang_vel_w;
+  a.terminated = terminated; a.truncated = truncated; a.pushed_ids = pushed_ids; a.n_pushed = n_pushed;
+  interval_step_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(a);
   CUDA_TRY(cudaGetLastError());
   return RL_OK;
 }

@@ -186,6 +186,41 @@ class MdpStepEngine:
         nat.check(self.lib.rl_contact_sensor_update(self._ctx, b.N, C.byref(fld), C.byref(st), t2h, float(dt),
                                                     float(force_threshold), int(ring_slot), self._stream()))
 
+    # ---- stage 8 of the step: the interval push event ----------------------------------------------------------
+    @staticmethod
+    def interval_event_cfg(term) -> nat.RlIntervalEventCfg:
+        """RlIntervalEventCfg of an interval ``push_by_setting_velocity`` term (``cfg.EventTermCfg``); a velocity key the
+        term does not name is the range (0, 0), as in push_by_setting_velocity [IL]."""
+        c = nat.RlIntervalEventCfg()
+        c.interval_lo, c.interval_hi = term.interval_range_s
+        vr = term.params.get("velocity_range", {})
+        for i, k in enumerate(("x", "y", "z", "roll", "pitch", "yaw")):
+            c.vel_lo[i], c.vel_hi[i] = vr.get(k, (0.0, 0.0))
+        return c
+
+    def interval_push(self, b: StateBuffers, cfg: nat.RlIntervalEventCfg, time_left: torch.Tensor,
+                      pushed_ids: torch.Tensor | None = None, n_pushed: torch.Tensor | None = None,
+                      env_ids: torch.Tensor | None = None, n_env_ids: torch.Tensor | None = None,
+                      dt: float | None = None, uniforms: torch.Tensor | None = None, seed: int = 0, step: int = 0,
+                      env_id_offset: int = 0, use_step_counter: bool = False) -> None:
+        """EventManager.reset(env_ids) [IL] with ``env_ids`` (timers of those envs resampled), otherwise
+        EventManager.apply("interval", dt) [IL] for the step just taken: timers of the envs the last ``step_pre_reset``
+        flagged done are resampled, every timer counts down ``dt`` (default: the spec's step_dt), the envs whose timer
+        ran out get ``root_lin_vel_w`` / ``root_ang_vel_w`` += U(velocity_range) and their ids land in
+        ``pushed_ids[:n_pushed]`` (int32 device tensors [N] / [1]). ``uniforms``: [8, N] U[0,1) instead of Philox."""
+        st = b.state_view()
+        rnd = b.random(seed, step, env_id_offset, False, use_step_counter)
+        dt = self.spec.step_dt if dt is None else dt
+        nat.check(self.lib.rl_interval_push(
+            self._ctx, b.N, C.byref(cfg), float(dt), time_left.data_ptr(), C.byref(st), b.terminated.data_ptr(),
+            b.truncated.data_ptr(), nat.ptr_of(env_ids), nat.ptr_of(n_env_ids), nat.ptr_of(pushed_ids),
+            nat.ptr_of(n_pushed), C.byref(rnd), nat.ptr_of(uniforms), self._stream()))
+
+    def reobserve(self, b: StateBuffers, env_ids: torch.Tensor, n_env_ids: torch.Tensor, **rng) -> None:
+        """The observation groups again for ``env_ids[:n_env_ids]`` only (the envs an interval push changed after the
+        fused post-reset launch observed them): the same rows a full observation pass would write."""
+        self.step(b, phases=nat.PHASE_OBS, env_ids=env_ids, n_env_ids=n_env_ids, **rng)
+
     # ---- the five entry points ----------------------------------------------------------------------
     def process_action(self, b: StateBuffers, with_target: bool = True, advance_step_counter: bool = True,
                        new_action: torch.Tensor | None = None) -> None:

@@ -9,7 +9,8 @@ play.py:175-248, scripts/tools/zero_agent.py:56-70): ``gym.make(id, cfg=env_cfg)
 ``env.action_manager`` (SURVEY.md 8(b).2) - those attributes exist here too, backed by the device buffers.
 
 In IsaacLab each manager loops over its terms in Python. Here ``env.step()`` is three CUDA launches
-(``rl_process_action`` -> state provider -> ``rl_step`` -> provider reset -> post-reset launch); the manager
+(``rl_process_action`` -> state provider -> ``rl_step`` -> provider reset -> post-reset launch), plus the interval push
+and a re-observation of the pushed envs when ``cfg.events`` enables it; the manager
 objects are views onto the buffers those launches fill, plus per-manager ``compute()`` entry points that run just
 their phase of the kernel. There is no CPU implementation behind any of this.
 
@@ -518,6 +519,76 @@ class ObservationManager(_ManagerBase):
         raise NotImplementedError("observation terms are evaluated inside the fused step; slice the group row instead")
 
 
+_VELOCITY_KEYS = ("x", "y", "z", "roll", "pitch", "yaw")
+
+
+def interval_push_terms(cfg) -> list[tuple[str, Any]]:
+    """The active terms of ``cfg.events``, checked against what this env runs on the device: at most one non-global
+    interval term calling ``push_by_setting_velocity`` [IL]. Anything else raises a ``ValueError`` naming the term -
+    reset events write physical state through ``ResetEventStateProvider``, startup events belong to the simulator."""
+    from .cfg import EventTermCfg
+    from .mdp import push_by_setting_velocity
+
+    events = getattr(cfg, "events", None)
+    terms = [(n, t) for n, t in events.items() if t is not None] if events is not None else []
+    for name, t in terms:
+        if not isinstance(t, EventTermCfg):
+            raise ValueError(f"event term '{name}': expected an EventTermCfg, got {type(t).__name__}")
+        if t.mode != "interval":
+            raise ValueError(f"event term '{name}': mode '{t.mode}' is not run by this env (reset events go through "
+                             "ResetEventStateProvider, startup events belong to the simulator); only mode='interval'")
+        if t.func is not push_by_setting_velocity:
+            raise ValueError(f"event term '{name}': interval function {getattr(t.func, '__name__', t.func)!r} is not "
+                             "supported; only push_by_setting_velocity")
+        if t.is_global_time:
+            raise ValueError(f"event term '{name}': is_global_time=True is not supported; only per-env interval timers")
+        rng = t.interval_range_s
+        if rng is None or len(rng) != 2 or not (float(rng[0]) <= float(rng[1])):
+            raise ValueError(f"event term '{name}': interval_range_s must be (lo, hi) with lo <= hi, got {rng!r}")
+        extra = set(t.params) - {"velocity_range", "asset_cfg"}
+        if extra:
+            raise ValueError(f"event term '{name}': unsupported params {sorted(extra)}")
+        asset = t.params.get("asset_cfg")
+        if asset is not None and getattr(asset, "name", None) != "robot":
+            raise ValueError(f"event term '{name}': only the 'robot' asset can be pushed")
+        vr = t.params.get("velocity_range", {})
+        bad = set(vr) - set(_VELOCITY_KEYS)
+        if bad:
+            raise ValueError(f"event term '{name}': unknown velocity_range keys {sorted(bad)}; known: {list(_VELOCITY_KEYS)}")
+        for k, (lo, hi) in vr.items():
+            if not float(lo) <= float(hi):
+                raise ValueError(f"event term '{name}': velocity_range['{k}'] needs lo <= hi, got {(lo, hi)!r}")
+    if len(terms) > 1:
+        raise ValueError(f"event terms {[n for n, _ in terms]}: one interval push term at most")
+    return terms
+
+
+class EventManager(_ManagerBase):
+    """EventManager [IL] surface for the event terms this env runs: the interval push (stage 8 of ``env.step()``,
+    ``rl_interval_push``). ``_interval_term_time_left`` holds one device timer tensor [N] per interval term, as
+    upstream; the env owns the tensors."""
+
+    def __init__(self, env, terms: list[tuple[str, Any]]):
+        super().__init__(env)
+        self._mode_term_names = {"interval": [n for n, _ in terms]} if terms else {}
+        self._mode_term_cfgs = {"interval": [t for _, t in terms]} if terms else {}
+        self._interval_term_time_left = [env.interval_time_left] if terms else []
+
+    @property
+    def available_modes(self) -> list[str]:
+        return list(self._mode_term_names)
+
+    @property
+    def active_terms(self) -> dict[str, list[str]]:
+        return dict(self._mode_term_names)
+
+    def get_term_cfg(self, name: str):
+        for names, cfgs in zip(self._mode_term_names.values(), self._mode_term_cfgs.values()):
+            if name in names:
+                return cfgs[names.index(name)]
+        raise ValueError(f"event term '{name}' not found")
+
+
 class _LazyLog(dict):
     """``extras["log"]``: a dict that fills itself from a snapshot of the device logging buffer on first access."""
 
@@ -617,6 +688,15 @@ class ManagerBasedRLEnv:
             self.was_on_pit = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
         self._all_ids = torch.arange(self.num_envs, dtype=torch.int32, device=self.device)
         self._n_all = torch.tensor([self.num_envs], dtype=torch.int32, device=self.device)
+        # interval push (stage 8, randomize_push_robot): per-env timers sampled now, like EventManager._prepare_terms [IL]
+        terms = interval_push_terms(cfg)
+        self._push_cfg = MdpStepEngine.interval_event_cfg(terms[0][1]) if terms else None
+        if terms:
+            self.interval_time_left = torch.zeros(self.num_envs, dtype=torch.float32, device=self.device)
+            self.pushed_ids = torch.zeros(self.num_envs, dtype=torch.int32, device=self.device)
+            self.n_pushed = torch.zeros(1, dtype=torch.int32, device=self.device)
+            self._reset_interval_timers()
+        self.event_manager = EventManager(self, terms)
         self._closed = False
 
     # -- properties the scripts / wrapper read --------------------------------------------------------
@@ -672,6 +752,20 @@ class ManagerBasedRLEnv:
         log["Metrics/base_velocity/error_vel_yaw"] = snap[kk + nat.RL_MAX_DONE_TERMS + 1]
         return log
 
+    def _push_rng(self) -> dict:
+        return dict(seed=self.seed, env_id_offset=self.rank * self.num_envs, use_step_counter=True)
+
+    def _reset_interval_timers(self) -> None:
+        """EventManager.reset(all ids) [IL]: fresh interval timers for every env."""
+        self.engine.interval_push(self.buffers, self._push_cfg, self.interval_time_left, env_ids=self._all_ids,
+                                  n_env_ids=self._n_all, **self._push_rng())
+
+    def _interval_push(self) -> None:
+        """Stage 8, event_manager.apply("interval") [IL]: after the command update, before the observations. The
+        pushed envs are ``pushed_ids[:n_pushed]`` - a simulator writes their root velocities into the simulation."""
+        self.engine.interval_push(self.buffers, self._push_cfg, self.interval_time_left, pushed_ids=self.pushed_ids,
+                                  n_pushed=self.n_pushed, **self._push_rng())
+
     def invalidate_derived(self) -> None:
         """Call after writing physical state into ``buffers`` by hand: the derived articulation views refresh lazily."""
         self._state_version += 1
@@ -684,6 +778,8 @@ class ManagerBasedRLEnv:
         b = self.buffers
         self.state_provider.advance(self)
         self.state_provider.reset(self, self._all_ids, self._n_all)
+        if self._push_cfg is not None:
+            self._reset_interval_timers()
         self._state_version += 1
         b.done_bits.zero_()
         self.engine.step(b, phases=nat.PHASE_RESET | nat.PHASE_COMMAND | nat.PHASE_OBS, env_ids=self._all_ids,
@@ -716,13 +812,21 @@ class ManagerBasedRLEnv:
             b.advance_log_slot()
             if nvtx:
                 torch.cuda.nvtx.range_push("mdp.step_post_reset")
+            push = self._push_cfg is not None
             if self.pit_grid is None:
                 eng.step_post_reset(b, **self._rng)                                      # 6b manager reset, 7 command, 9 obs
+                if push:   # 8 after the fused launch: the pushed envs' observation rows are written again
+                    self._interval_push()
+                    eng.reobserve(b, self.pushed_ids, self.n_pushed, **self._rng)
             else:   # the pit branch of _update_command sits between the command update and the observations
                 rng = self._rng
                 eng.step(b, phases=nat.PHASE_RESET | nat.PHASE_COMMAND, **rng)
                 eng.command_pit_restrict(b, self.pit_grid, self.was_on_pit, **rng)
+                if push:
+                    self._interval_push()                                                # 8
                 eng.step(b, phases=nat.PHASE_OBS, **rng)
+            if push:
+                self._state_version += 1
             if nvtx:
                 torch.cuda.nvtx.range_pop()
         finally:

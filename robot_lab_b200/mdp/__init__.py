@@ -107,6 +107,18 @@ terrain_out_of_bounds = _make("done", "terrain_out_of_bounds", "terrain_out_of_b
 illegal_contact = _make("done", "illegal_contact", "illegal_contact", f"{_IL} terminations.illegal_contact")
 
 
+# --- event terms ------------------------------------------------------------------------------------------
+# Not in the registry above: an event term is no term of the fused step. The env recognises this marker in
+# ``cfg.events`` and runs it as ``rl_interval_push`` (stage 8 of the step); calling it directly is an error.
+def push_by_setting_velocity(env, env_ids, velocity_range, asset_cfg=None):
+    """push_by_setting_velocity [IL] (isaaclab.envs.mdp.events): root_vel_w[env_ids] += U(velocity_range). Runs on the
+    device inside ``env.step()`` when configured as an interval event term (``ManagerBasedRLEnv`` / EventManager)."""
+    raise NotImplementedError("push_by_setting_velocity runs inside env.step() as an interval event term (cfg.events)")
+
+
+push_by_setting_velocity.rl_kind = "event"
+
+
 def get(name: str) -> Callable:
     return _REGISTRY[name]
 

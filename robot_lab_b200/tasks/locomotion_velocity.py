@@ -8,7 +8,10 @@ Per-robot files (``unitree.py`` next to this one) then set weights and names exa
 ``rough_env_cfg.py`` / ``flat_env_cfg.py`` override chains do.
 
 Events (startup / reset randomisation) and curricula are physics-side or host-side pieces outside the MDP step
-(SURVEY.md section 2 rows 5-6); they are not represented here.
+(SURVEY.md section 2 rows 5-6); they are not represented here, with one exception: the interval push
+``randomize_push_robot`` (V/velocity_env_cfg.py:366-371), stage 8 of the env step. ``cfg.events.randomize_push_robot``
+is None (off) by default, so every task keeps the step without pushes; ``push_robot_event_term()`` returns the
+reference's term, which the reference has on by default.
 """
 
 from __future__ import annotations
@@ -21,6 +24,7 @@ from ..assets import RobotAsset
 from ..cfg import (
     AdditiveUniformNoiseCfg as Unoise,
     ContactSensorCfg,
+    EventTermCfg as EventTerm,
     JointPositionActionCfg,
     ObservationGroupCfg as ObsGroup,
     ObservationTermCfg as ObsTerm,
@@ -145,6 +149,18 @@ def _obs_group(corrupt: bool) -> ObsGroup:
     return g
 
 
+def push_robot_event_term(interval_range_s: tuple[float, float] = (10.0, 15.0),
+                          velocity_range: dict | None = None) -> EventTerm:
+    """The reference's ``randomize_push_robot`` (V/velocity_env_cfg.py:366-371): push_by_setting_velocity every 10 to
+    15 s per env. The term, its function and the interval are the reference's (SURVEY.md section 3.2, stage 8); the
+    x / y range of +-0.5 m/s is the value of the IsaacLab locomotion velocity template that file follows
+    (isaaclab_tasks .../locomotion/velocity/velocity_env_cfg.py, ``push_robot``), not read from the reference itself."""
+    if velocity_range is None:
+        velocity_range = {"x": (-0.5, 0.5), "y": (-0.5, 0.5)}
+    return EventTerm(func=mdp.push_by_setting_velocity, mode="interval", interval_range_s=interval_range_s,
+                     params={"velocity_range": velocity_range})
+
+
 class LocomotionVelocityRoughEnvCfg:
     """Base task cfg (V/velocity_env_cfg.py:695-743)."""
 
@@ -170,6 +186,8 @@ class LocomotionVelocityRoughEnvCfg:
             illegal_contact=DoneTerm(func=mdp.illegal_contact,
                                      params={"sensor_cfg": _contacts(body_names=""), "threshold": 1.0}),
         )
+        # interval events: off by default (the reference enables randomize_push_robot; push_robot_event_term() is it)
+        self.events = TermContainer(randomize_push_robot=None)
         self.decimation = 4
         self.episode_length_s = 20.0
         self.sim.dt = 0.005
